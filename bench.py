@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the LightGlue matcher forward path on B200 (contract: see the task brief).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload at N GPUs: BASELINE.json configs[1] on every GPU -- SuperPoint-shaped synthetic pairs,
@@ -29,6 +29,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -118,6 +119,44 @@ class ClockSampler:
         return {"sm_mhz": statistics.median(sm), "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_outputs(res: dict, out_dir: str, cap_bytes: int = 64 << 20) -> None:
+    """Write the output dict of one forward as `out_dir/<name>.npy`: floating outputs as float32, integer outputs (match
+    indices, exit layers) as float64, which holds them exactly.  A per-pair list (`matches`, `scores`, `stops`) is written
+    concatenated, its tensors' lengths as `<name>_lengths.npy`.  Above `cap_bytes` in all, only a fixed seeded sample of
+    the pairs is written, their indices as `pairs.npy`."""
+    b = res["matches0"].shape[0]
+
+    def arrays(sel):
+        out = {}
+        for k, v in res.items():
+            if isinstance(v, list) and len(v) == b:
+                parts = [v[i] for i in sel]
+                if parts and torch.is_tensor(parts[0]):
+                    out[k] = torch.cat([p.cpu() for p in parts])
+                    out[k + "_lengths"] = torch.tensor([len(p) for p in parts])
+                else:
+                    out[k] = torch.tensor(parts)
+            elif torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == b:
+                out[k] = v[sel].cpu()
+            else:
+                out[k] = torch.as_tensor(v)
+        return {k: t.to(torch.float32 if t.is_floating_point() else torch.float64).numpy() for k, t in out.items()}
+
+    sel = list(range(b))
+    arr = arrays(sel)
+    if sum(a.nbytes for a in arr.values()) > cap_bytes:
+        order = torch.randperm(b, generator=torch.Generator().manual_seed(0)).tolist()
+        k = b
+        while k > 1 and sum(a.nbytes for a in arr.values()) > cap_bytes:
+            k = max(1, k * 3 // 4)
+            sel = sorted(order[:k])
+            arr = arrays(sel)
+        arr["pairs"] = torch.tensor(sel, dtype=torch.float64).numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arr.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def host_cores() -> int:
     n = os.cpu_count() or 1
     try:
@@ -185,11 +224,11 @@ class CpuReference:
         return best
 
     def run(self, n_pairs: int, budget_s: float = 1e9):
-        """Returns (pairs done, seconds)."""
+        """Returns (pairs done, seconds); the output of the last forward is kept as `last`."""
         done, t0 = 0, time.perf_counter()
         with torch.no_grad():
             while done < n_pairs:
-                self.fwd(self.data)
+                self.last = self.fwd(self.data)
                 done += self.pairs_per_forward
                 if time.perf_counter() - t0 > budget_s:
                     break
@@ -222,6 +261,8 @@ def run_reference(args, rank: int):
         n_steps += 1
         if time.perf_counter() - t_all > 100:
             break
+    if args.dump_outputs:
+        dump_outputs(cpu.last, args.dump_outputs)
     value = done / secs
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "pairs/s", "n_gpus": args.gpus,
@@ -320,7 +361,11 @@ def main():
     ap.add_argument("--no-other-mode", action="store_true")
     ap.add_argument("--no-extractor", action="store_true")
     ap.add_argument("--profile", action="store_true", help="2 forwards and exit (for ncu; prints nothing timed)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0's pairs; inputs are seeded)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -438,6 +483,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
     value = world * B * args.steps / (ms / 1000.0)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- timed region 2: end to end through the public API with pinned host inputs
     from lightglue_b200.pipeline import match_stream
@@ -452,7 +499,7 @@ def main():
 
     run_e2e(4)  # warm-up: also allocates the three pinned result slots of match_stream
     barrier()
-    e2s = max(3, args.steps)
+    e2s = args.steps
     e0.record()
     res = run_e2e(e2s)
     e1.record()

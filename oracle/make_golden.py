@@ -1,6 +1,6 @@
 """Generate tests/golden/*.pt by running the UNMODIFIED reference matcher in this container.
 
-    python oracle/make_golden.py            # needs /root/reference (read-only); CPU, fp32
+    python oracle/make_golden.py [batch_semantics]   # needs the reference checkout (REF); CPU, fp32
 
 The reference package cannot be imported as a package here (``import lightglue`` pulls kornia, which
 is absent), but ``lightglue/lightglue.py`` only needs numpy + torch, so it is loaded by file path
@@ -70,11 +70,46 @@ def build_inputs(rc: dict):
     return data, perm, sd
 
 
+def batch_semantics(ref) -> None:
+    """batch_early_exit.pt: the reference's adaptive depth on B=2 batches (tests/test_reference_batch_semantics.py).
+    Weights with which pair 41 exits early alone and pair 42 does not; outputs of each pair alone, of pair 41 twice in
+    one batch and of the two together."""
+    rc = dict(weight_seed=2, n=192, seeds=(41, 42), depth_confidence=0.95, width_confidence=-1)
+    sd = synth.make_state_dict(adaptive=True, seed=rc["weight_seed"])
+    model = ref.LightGlue(features=None, depth_confidence=rc["depth_confidence"],
+                          width_confidence=rc["width_confidence"]).eval()
+    missing, unexpected = model.load_state_dict(sd, strict=False)
+    assert not unexpected and all(k == "confidence_thresholds" for k in missing), (missing, unexpected)
+    p41, p42 = (synth.make_pair(rc["n"], b=1, seed=s)[0] for s in rc["seeds"])
+
+    def cat(pairs):
+        return {k: {kk: torch.cat([p[k][kk] for p in pairs]) for kk in pairs[0][k]} for k in ("image0", "image1")}
+
+    outs = {}
+    for name, data in (("alone41", p41), ("alone42", p42), ("twice41", cat([p41, p41])), ("mixed", cat([p41, p42]))):
+        out = model(data)
+        outs[name] = {"stop": int(out["stop"]), "matches0": out["matches0"].to(torch.int32),
+                      "matches1": out["matches1"].to(torch.int32), "matching_scores0": out["matching_scores0"],
+                      "matching_scores1": out["matching_scores1"]}
+        print(f"batch_early_exit/{name:8s} stop={outs[name]['stop']}")
+    fix = {
+        "recipe": rc,
+        "weights_checksum": {k: synth.checksum(v) for k, v in list(sd.items())[:4]},
+        "inputs_checksum": {s: {"k0": synth.checksum(p["image0"]["keypoints"]), "d1": synth.checksum(p["image1"]["descriptors"])}
+                            for s, p in zip(rc["seeds"], (p41, p42))},
+        "out": outs,
+    }
+    torch.save(fix, os.path.join(OUT, "batch_early_exit.pt"))
+
+
 def main() -> None:
     torch.set_grad_enabled(False)
     torch.set_num_threads(os.cpu_count() or 1)
     ref = load_reference()
     os.makedirs(OUT, exist_ok=True)
+    batch_semantics(ref)
+    if sys.argv[1:] == ["batch_semantics"]:
+        return
     for name, rc in CASES.items():
         data, perm, sd = build_inputs(rc)
         conf = conf_of(rc)

@@ -8,7 +8,8 @@ covers (grayscale input, ``forward``), so the generator provides stand-ins for e
 ``kornia.color`` stub that must never be called, a minimal ``Extractor`` base that only builds ``self.conf`` the
 way utils.py:131-134 does, and a ``torch.hub.load_state_dict_from_url`` that returns the seeded synthetic weights
 (oracle/superpoint_synth.py) -- and loads the reference file by path.  Everything else that runs is the
-reference's own code.  Fixtures store the recipe, checksums of the regenerated image / weights and the outputs.
+reference's own code.  Fixtures store the recipe, checksums of the regenerated image / weights and the outputs;
+``float64/<name>.pt`` holds the keypoints and scores of the same forward in float64.
 """
 from __future__ import annotations
 
@@ -74,6 +75,7 @@ def main():
     ref = load_reference(weights)
     os.makedirs(OUT, exist_ok=True)
     only = set(sys.argv[1:])  # optional: names of the cases to (re)generate
+    grid_sample = torch.nn.functional.grid_sample
     for name, rc in CASES.items():
         if only and name not in only:
             continue
@@ -85,6 +87,16 @@ def main():
             # keep the fixtures small: above 600 keypoints only every 4th descriptor row is stored
             res["desc_stride"] = [4 if t.shape[0] > 600 else 1 for t in res["descriptors"]]
             res["descriptors"] = [t[::st].clone() for t, st in zip(res["descriptors"], res["desc_stride"])]
+            # The same forward in float64 (float64/<name>.pt: keypoints and scores): fp32 scores depend on the
+            # convolutions' summation order, which varies with the host CPU and thread count by more than the oracle
+            # test's tolerance; float64 scores do not.  superpoint.py:210 casts the keypoints to float32, so the sampling
+            # grid is cast to the descriptor map's dtype.
+            torch.nn.functional.grid_sample = lambda inp, grid, *a, **k: grid_sample(inp, grid.to(inp.dtype), *a, **k)
+            try:
+                out64 = model.double()({"image": image.double()})
+            finally:
+                torch.nn.functional.grid_sample = grid_sample
+            res64 = {k: [t.clone() for t in out64[k]] for k in ("keypoints", "keypoint_scores")}
         else:
             raise ValueError("batched cases need max_num_keypoints (the reference stacks per-image results)")
         fix = {
@@ -95,6 +107,8 @@ def main():
             "out": res,
         }
         torch.save(fix, os.path.join(OUT, name + ".pt"))
+        os.makedirs(os.path.join(OUT, "float64"), exist_ok=True)
+        torch.save(res64, os.path.join(OUT, "float64", name + ".pt"))
         print(name, [tuple(t.shape) for t in res["keypoints"]], [tuple(t.shape) for t in res["descriptors"]], "max score", float(max(t.max() for t in res["keypoint_scores"])))
 
 

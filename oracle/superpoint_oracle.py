@@ -69,7 +69,7 @@ def sample_descriptors(kpts_xy: torch.Tensor, dense: torch.Tensor, cell: int = C
     k = kpts_xy - cell / 2 + 0.5
     k = k / torch.tensor([wc * cell - cell / 2 - 0.5, hc * cell - cell / 2 - 0.5]).to(k)
     k = k * 2 - 1
-    out = F.grid_sample(dense[None], k.view(1, 1, -1, 2), mode="bilinear", align_corners=True)
+    out = F.grid_sample(dense[None], k.view(1, 1, -1, 2).to(dense), mode="bilinear", align_corners=True)
     return F.normalize(out.reshape(c, -1), p=2, dim=0).t().contiguous()
 
 

@@ -6,8 +6,9 @@ import torch
 from lightglue_b200 import synth
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-# matcher fixtures only (sp_* are the SuperPoint extractor oracle's, tests/test_superpoint_oracle_golden.py)
-ALL_CASES = sorted(f[:-3] for f in os.listdir(GOLDEN) if f.endswith(".pt") and not f.startswith("sp_"))
+# matcher fixtures only (sp_* are the SuperPoint extractor oracle's, tests/test_superpoint_oracle_golden.py; batch_* hold
+# the reference's B > 1 semantics, tests/test_reference_batch_semantics.py)
+ALL_CASES = sorted(f[:-3] for f in os.listdir(GOLDEN) if f.endswith(".pt") and not f.startswith(("sp_", "batch_")))
 
 
 def load_case(name):
