@@ -14,8 +14,6 @@
 // Warp roles (384 threads = 3 warpgroups): warpgroup 0 = {warp 0 TMA producer, warp 1 TMEM owner + MMA issuer of
 // tile 0, warp 2 MMA issuer of tile 1, 1 idle warp} shrinks its registers (setmaxnreg.dec); warpgroups 1 and 2 are
 // the softmax warpgroups of query tile 0 / 1 (one query row per thread; warp w reads TMEM lanes 32*(w%4)..).
-#include <stdlib.h>
-
 #include "lg_handle.h"
 #include "tc_common.cuh"
 
@@ -36,7 +34,6 @@ struct AttnParams {
   __nv_bfloat16* ctxh; __nv_bfloat16* ctxl;
   int kv_shift;
   int rows_per_cta;  // 256 (two query tiles per CTA) or 128 (one: small problems that would not fill the SMs)
-  int pingpong;      // alternate the exponential phases of the CTA's two query tiles (LG_ATTN_NO_PINGPONG=1 switches it off)
   SeqState st;
   unsigned int* dbg;
 };
@@ -121,7 +118,7 @@ __device__ __forceinline__ void softmax_tile(const AttnParams& p, int t, int nt,
         //    double buffering: four resident tiles that wait for their MMAs beat two that do not.
         //  (tools/micro/micro_exp.cu: the exponential phase alone runs at 9.8 cycles per MUFU with one warp per scheduler and
         //  8.2 with two -- the 8-cycle MUFU issue rate -- so the phase itself is not what is slow.)
-        const bool pingpong = nt > 1 && p.pingpong;
+        const bool pingpong = nt > 1;
         // One token per SCHEDULER: the warp of tile 0 and the warp of tile 1 that own the same row quarter share a
         // scheduler and its MUFU; named barrier 2 + 2 q + t (64 threads) hands the exponential phase from one to the other,
         // so a hand-over never waits for the slowest of the four schedulers (a CTA-wide token, barriers 2 / 3 with 256
@@ -407,8 +404,6 @@ int tc_attention(LgHandle* h, const TcBuffers& b, const SeqState& st, int kv_shi
   AttnParams p;
   p.q_map = c->qm; p.k_map = c->km; p.vt_map = c->vm;
   p.ctxh = b.ctxh; p.ctxl = b.ctxl; p.kv_shift = kv_shift; p.st = st; p.dbg = h->tc.dbg;
-  const char* npp = getenv("LG_ATTN_NO_PINGPONG");
-  p.pingpong = (npp && atoi(npp) != 0) ? 0 : 1;
   dim3 grid((st.Lp + 2 * QT - 1) / (2 * QT), LG_HEADS, st.S);
   p.rows_per_cta = 2 * QT;
   if ((long)grid.x * grid.y * grid.z < 2 * lg_num_sms()) {  // fewer CTAs than resident slots: one query tile per CTA instead
@@ -420,11 +415,9 @@ int tc_attention(LgHandle* h, const TcBuffers& b, const SeqState& st, int kv_shi
   cudaLaunchConfig_t cfg{};
   cudaLaunchAttribute at[1];
   cfg.gridDim = grid; cfg.blockDim = dim3(384); cfg.dynamicSmemBytes = smem2; cfg.stream = stream;
-  if (tc_use_pdl()) {
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-  }
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = 1;
   const cudaError_t e = cudaLaunchKernelEx(&cfg, tc_attention2_kernel, p);
   if (e != cudaSuccess) return lg_set_cuda_error(e, __FILE__, __LINE__);
   return 0;

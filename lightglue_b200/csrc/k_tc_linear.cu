@@ -2,8 +2,8 @@
 //
 //   C[128 rows, 256 cols per accumulator slot] = A[rows, K] * W[cols, K]^T     (fp32 accumulate in TMEM)
 //
-// * operands are bf16, K-major; tiles are staged by TMA (128-byte swizzle) into a shared-memory ring,
-//   a single elected thread issues tcgen05.mma (M=128, N=256, K=16), tcgen05.commit releases the ring
+// * operands are bf16, K-major; tiles are staged by TMA (128-byte swizzle) into a shared-memory ring, one elected
+//   thread of a CTA pair issues tcgen05.mma (M=256 over the pair, N=256, K=16), tcgen05.commit releases the ring
 //   slot and finally signals the epilogue warps, which read the accumulator back with tcgen05.ld;
 // * LG_PREC_BF16X3 runs three passes over K into the same accumulator: A_lo*W_hi + A_hi*W_lo +
 //   A_hi*W_hi with x = hi + lo, hi = bf16(x), lo = bf16(x - hi)  (~16 mantissa bits per operand);
@@ -14,7 +14,6 @@
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2-5 = epilogue
 // (warp w reads TMEM lanes 32*(w%4) .. +31, one accumulator row per thread).
 #include <stdio.h>
-#include <stdlib.h>
 
 #include <unordered_map>
 
@@ -29,12 +28,11 @@ constexpr int BM = 128, BN = 256, BK = 64;
 constexpr int A_TILE_BYTES = BM * BK * 2;  // 16 KB
 constexpr int W_TILE_BYTES = BN * BK * 2;  // 32 KB
 
-enum { TEPI_QKV = 0, TEPI_BF16 = 1, TEPI_LN_GELU = 2, TEPI_RESID = 3, TEPI_F32 = 4, TEPI_LSE = 5, TEPI_ARGMAX = 6, TEPI_CONV = 7 };
+enum { TEPI_QKV = 0, TEPI_LN_GELU = 2, TEPI_RESID = 3, TEPI_F32 = 4, TEPI_LSE = 5, TEPI_ARGMAX = 6, TEPI_CONV = 7 };
 
 struct TcLinParams {
   CUtensorMap a_hi[2], a_lo[2];  // A segment 0 / 1
-  CUtensorMap w_hi, w_lo;        // 3-D: (K, Nout, select), box 64 x 256 rows
-  CUtensorMap w_hi_half, w_lo_half;  // same tensors, box 64 x 128 rows: each CTA of a pair holds one half of the N tile (cta_group::2)
+  CUtensorMap w_hi, w_lo;        // 3-D: (K, Nout, select), box 64 x 128 rows (mma_n / 2): each CTA of a pair holds one half of the N tile
   int kb0, kb_total, passes, n_tiles;
   int epi, rope;
   SeqState st;
@@ -57,7 +55,7 @@ struct TcLinParams {
   // pixels again on the way out (conv_w2 = W + 2, conv_plane = (H+2)(W+2), conv_rows = B conv_plane) and applies ReLU.
   int conv_cb, conv_w2, conv_h, conv_w, relu;
   long conv_plane, conv_rows;
-  int mma_n;  // pair mode only: N of the MMAs when fewer than 256 output columns exist (64 / 128; 0 = 256): each CTA then
+  int mma_n;  // N of the MMAs when fewer than 256 output columns exist (64 / 128; 0 = 256): each CTA then
               // holds mma_n / 2 rows of the W tile and the accumulator uses the first mma_n columns of its slot
   // epilogue tensor maps (all boxes are 32 rows x 128 bytes, 128B swizzle)
   CUtensorMap o_h;          // bf16 hi output [rows, ldb], box 64 cols x 32 rows, 128B swizzle (two chunks per store)
@@ -78,17 +76,14 @@ struct TcLinParams {
 // x 16 B per row) -> coalesced global loads / stores.
 // ------------------------------------------------------------------------------------------------
 
-// CG2: CTA pairs (cta_group::2).  The two CTAs of a cluster take the two row tiles of a "tile pair" with the same
+// CTA pairs (cta_group::2).  The two CTAs of a cluster take the two row tiles of a "tile pair" with the same
 // n-tile; one thread of the leader CTA issues M=256 MMAs that read A (128 rows) and HALF of the W tile (128 of its
-// 256 rows) from each CTA's shared memory, so every SM receives only half of the weight bytes, a ring stage is
-// 32 KB instead of 48 and more stages fit.  X3 (CG2 only): split-bf16 with the K block outermost -- one stage holds
-// A_hi, A_lo, W_hi, W_lo of a 64-wide K block and feeds all three passes (A_lo W_hi, A_hi W_lo, A_hi W_hi): the
-// W_hi / A_hi tiles are loaded once instead of twice.  With two accumulator slots (LayerNorm variant) the slots
-// take consecutive stages of the same format.  Non-CG2 (per-tile weight selection: final_proj heads, assignment
-// sweeps): one CTA per tile, passes outermost, as in round 1.
-template <int NSLOT, bool CG2, bool X3>
+// 256 rows) from each CTA's shared memory, so every SM receives only half of the weight bytes and a ring stage is
+// 32 KB.  X3: split-bf16 with the K block outermost -- one stage holds A_hi, A_lo, W_hi, W_lo of a 64-wide K block
+// and feeds all three passes (A_lo W_hi, A_hi W_lo, A_hi W_hi): the W_hi / A_hi tiles are loaded once instead of
+// twice.  With two accumulator slots (LayerNorm variant) the slots take consecutive stages of the same format.
+template <int NSLOT, bool X3>
 struct LinCfg {
-  static_assert(CG2 || !X3, "the K-outer split staging exists in the CTA-pair kernels only");
   // accumulator hand-over barriers: NSLOT == 1: two 256-column buffers used by alternate tiles; NSLOT == 2 (LayerNorm):
   // the two 256-column SLOTS of one tile, completed and released one after the other
   static constexpr int NBUF = 2;
@@ -99,19 +94,16 @@ struct LinCfg {
   // control warps ahead of the epilogue warps: TMA producer, MMA issuer
   static constexpr int CTRL = 2;
   static constexpr int THREADS = (CTRL + EW) * 32;
-  static constexpr int W_PART = CG2 ? W_TILE_BYTES / 2 : W_TILE_BYTES;  // bytes of one W tile held by this CTA
-  static constexpr int STAGE_BYTES = CG2 ? (X3 ? 2 * A_TILE_BYTES + 2 * W_PART : A_TILE_BYTES + W_PART)
-                                         : A_TILE_BYTES + NSLOT * W_TILE_BYTES;
+  static constexpr int W_PART = W_TILE_BYTES / 2;  // bytes of one W tile held by this CTA
+  static constexpr int STAGE_BYTES = X3 ? 2 * A_TILE_BYTES + 2 * W_PART : A_TILE_BYTES + W_PART;
   static constexpr int COLS = NSLOT * BN;
   // per epilogue warp: box A (4 KB: fp32 32x32 output box / rotary cos), box B (4 KB: 16-bit 32x64 box, hi or
   // fp16), box C (4 KB: rotary sin, or the dense 32x32 bf16 "lo" box).  The LayerNorm variant has no box A.
   // (NSLOT == 2: one dense 32x32 bf16 box, 2 KB, shared by the hi and lo images)
-  // (NSLOT == 2: dense 32x32 bf16 boxes of 2 KB: one shared by the hi and lo images, or -- pair kernels -- one each)
   static constexpr int WARP_BYTES = NSLOT == 1 ? 3 * 4096 : 2048;
   // LayerNorm variant: 16 of the 64 slot-0 values every epilogue thread keeps across the MMAs of slot 1 live in shared
-  // memory, the other 48 in registers (576 threads leave 96 registers per thread); the single-CTA debug variant has no
-  // room for it next to its 80 KB stages and spills instead
-  static constexpr int STASH_SMEM = (NSLOT == 2 && CG2) ? 16 : 0;
+  // memory, the other 48 in registers (576 threads leave 96 registers per thread)
+  static constexpr int STASH_SMEM = NSLOT == 2 ? 16 : 0;
   static constexpr int STASH_BYTES = STASH_SMEM * EW * 32 * 4;
   static constexpr int BOXB_OFF = NSLOT == 1 ? 4096 : 0;
   static constexpr int BOXC_OFF = NSLOT == 1 ? 8192 : 0;
@@ -138,17 +130,29 @@ __device__ __forceinline__ float ex2_approx(float x) {
 template <int NTHREADS>
 __device__ __forceinline__ void epi_bar_n() { asm volatile("bar.sync 1, %0;" ::"n"(NTHREADS) : "memory"); }  // the epilogue warps
 
+// Row tiles ("slots") per sequence.  With per-tile weight selection the two CTAs of a pair share one W tile, so a pair
+// must not straddle two sequences: an odd tile count gets one more slot, a dead tile past the sequence's end (its A rows
+// are the next sequence's or TMA zero fill; its epilogue stores nothing).  Without weight selection pairs may cross.
+__host__ __device__ __forceinline__ int row_slots(const SeqState& st, int w_select) {
+  const int tiles = st.Lp / BM;
+  return tiles + (w_select != 0 && tiles % 2 != 0);
+}
+// tiles of the launch; S is even, so they come in pairs
+__host__ __device__ __forceinline__ int total_tiles(const TcLinParams& p) {
+  return p.n_tiles * p.st.S * row_slots(p.st, p.w_select);
+}
+
 struct TileInfo {
   int s, r0, n_tile, sel, len;
   long grow0;
 };
 // decode tile t (n-tile fastest); returns false for tiles with nothing to do (all fields are filled either way)
 __device__ __forceinline__ bool decode_tile(const TcLinParams& p, int t, int n_tiles, TileInfo& ti) {
-  const int tiles_per_seq = p.st.Lp / BM;
+  const int slots = row_slots(p.st, p.w_select);
   ti.n_tile = t % n_tiles;
   const int rt = t / n_tiles;
-  ti.s = rt / tiles_per_seq;
-  ti.r0 = (rt % tiles_per_seq) * BM;
+  ti.s = rt / slots;
+  ti.r0 = (rt % slots) * BM;
   ti.len = p.st.len[ti.s];
   ti.grow0 = (long)ti.s * p.st.Lp + ti.r0;
   ti.sel = 0;
@@ -163,47 +167,35 @@ __device__ __forceinline__ bool decode_tile(const TcLinParams& p, int t, int n_t
   return live;
 }
 
-// Tile schedule.  Plain mode: CTA c walks tiles c, c + grid, ...  Pair mode (MC == CG2): the two CTAs of a cluster
-// take the two row tiles of a "tile pair" with the same n-tile; both walk the same list.
-template <bool MC>
+// Tile schedule: the two CTAs of a cluster take the two row tiles of a "tile pair" with the same n-tile; both walk
+// the same list of tile pairs.
 struct TileWalk {
   int cur, step, end, rank, n_tiles;
   __device__ TileWalk(int total_tiles, int n_tiles_) : n_tiles(n_tiles_) {
-    if (MC) {
-      rank = (int)cluster_ctarank();
-      cur = blockIdx.x / 2; step = gridDim.x / 2; end = total_tiles / 2;  // tile pairs (row tiles come in pairs: S is even)
-    } else {
-      rank = 0; cur = blockIdx.x; step = gridDim.x; end = total_tiles;
-    }
+    rank = (int)cluster_ctarank();
+    cur = blockIdx.x / 2; step = gridDim.x / 2; end = total_tiles / 2;
   }
-  // returns false when done; `mine` = this CTA's tile (decoded), `run` = the CTA must run loads + MMAs,
-  // `store` = its epilogue may write
+  // returns false when done; `mine` = this CTA's tile (decoded), `store` = its epilogue may write (the pair runs loads
+  // and MMAs as long as either tile is live)
   __device__ bool next(const TcLinParams& p, TileInfo& mine, bool& store) {
     while (cur < end) {
       const int id = p.reverse ? end - 1 - cur : cur;
       cur += step;
-      if (MC) {
-        const int n_tile = id % n_tiles, rtp = id / n_tiles;
-        TileInfo peer;
-        const bool lm = decode_tile(p, (rtp * 2 + rank) * n_tiles + n_tile, n_tiles, mine);
-        const bool lp = decode_tile(p, (rtp * 2 + (rank ^ 1)) * n_tiles + n_tile, n_tiles, peer);
-        if (!lm && !lp) continue;
-        store = lm;
-        return true;
-      } else {
-        if (!decode_tile(p, id, n_tiles, mine)) continue;
-        store = true;
-        return true;
-      }
+      const int n_tile = id % n_tiles, rtp = id / n_tiles;
+      TileInfo peer;
+      const bool lm = decode_tile(p, (rtp * 2 + rank) * n_tiles + n_tile, n_tiles, mine);
+      const bool lp = decode_tile(p, (rtp * 2 + (rank ^ 1)) * n_tiles + n_tile, n_tiles, peer);
+      if (!lm && !lp) continue;
+      store = lm;
+      return true;
     }
     return false;
   }
 };
 
-template <int NSLOT, int EPI, bool CG2, bool X3>
-__global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_kernel(const __grid_constant__ TcLinParams p) {
-  using C = LinCfg<NSLOT, CG2, X3>;
-  constexpr bool MC = CG2;
+template <int NSLOT, int EPI, bool X3>
+__global__ void __launch_bounds__(LinCfg<NSLOT, X3>::THREADS, 1) tc_linear_kernel(const __grid_constant__ TcLinParams p) {
+  using C = LinCfg<NSLOT, X3>;
   constexpr int EPI_WARPS = C::EW;
   auto epi_bar = [] { epi_bar_n<C::EW * 32>(); };
   constexpr int STAGES = C::STAGES, NBUF = C::NBUF, STAGE_BYTES = C::STAGE_BYTES, COLS = C::COLS;
@@ -226,34 +218,30 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
 
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
   const int n_tiles = p.n_tiles;
-  const int total_tiles = n_tiles * p.st.S * (p.st.Lp / BM);
-  // ring iterations per tile: pair mode = (K block, accumulator slot), split-bf16 passes inside an iteration;
-  // plain mode = (pass, K block), all slots inside an iteration
-  const int iters = CG2 ? p.kb_total * NSLOT : p.passes * p.kb_total;
-  const int rank = CG2 ? (int)cluster_ctarank() : 0;
+  const int tiles = total_tiles(p);
+  // ring iterations per tile: (K block, accumulator slot), split-bf16 passes inside an iteration
+  const int iters = p.kb_total * NSLOT;
+  const int rank = (int)cluster_ctarank();
 
   pdl_launch_dependents();  // the next kernel's CTAs may take this SM as soon as this CTA has left it
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&p.a_hi[0]);
     tma_prefetch_desc(&p.w_hi);
-    // pair mode: only the leader's `full` / `acc_empty` barriers are waited on (its TMA bytes AND the peer's complete
-    // there; both CTAs' epilogue warps arrive there); `empty` / `acc_full` exist in both CTAs and receive the leader's
-    // multicast commits
+    // only the leader's `full` / `acc_empty` barriers are waited on (its TMA bytes AND the peer's complete there; both
+    // CTAs' epilogue warps arrive there); `empty` / `acc_full` exist in both CTAs and receive the leader's multicast
+    // commits
     for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-    for (int i = 0; i < NBUF; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], (CG2 ? 2 : 1) * EPI_WARPS); }
+    for (int i = 0; i < NBUF; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 2 * EPI_WARPS); }
     for (int i = 0; i < EPI_WARPS; ++i) mbar_init(&ldbar[i], 1);
     fence_barrier_init();
   }
-  if (warp == 1) {
-    if (CG2) tmem_alloc_cg2<512>(tmem_slot);
-    else tmem_alloc<512>(tmem_slot);
-  }
+  if (warp == 1) tmem_alloc_cg2<512>(tmem_slot);
   if (EPI == TEPI_LN_GELU && warp >= C::CTRL) {
     for (int i = threadIdx.x - C::CTRL * 32; i < COLS; i += EPI_WARPS * 32) { s_gamma[i] = p.ln_g[i]; s_beta[i] = p.ln_b[i]; }
   }
   tc_fence_before();
   __syncthreads();
-  if (MC) cluster_sync_all();  // the peer's barriers are initialised before anything can arrive on them
+  cluster_sync_all();  // the peer's barriers are initialised before anything can arrive on them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   // everything above (barriers, TMEM, descriptor prefetch, LayerNorm vectors = weights) overlapped the tail of the
@@ -264,7 +252,7 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
     // ------------------------------------------------------------------ TMA producer
     if (elect_one()) {
       int g = 0;  // global k-block counter across tiles (ring position)
-      TileWalk<MC> walk(total_tiles, n_tiles);
+      TileWalk walk(tiles, n_tiles);
       TileInfo ti;
       bool store;
       while (walk.next(p, ti, store)) {
@@ -272,82 +260,57 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
           const int stage = g % STAGES, round = g / STAGES;
           mbar_wait(&empty[stage], (round & 1) ^ 1, p.dbg, 17, it);
           uint8_t* sa = smem + stage * STAGE_BYTES;
-          if (CG2) {
-            // pair mode: this CTA's A rows and its half (128 of 256 rows) of the W tile; the bytes of BOTH CTAs complete
-            // on the leader's barrier, which only the leader arms
-            const int sl_ = it / p.kb_total, kb = it % p.kb_total;  // slot outermost: slot 0 completes (and is normalised) first
-            int seg = kb >= p.kb0 ? 1 : 0;
-            int kc = (seg ? kb - p.kb0 : kb) * BK;
-            int arow = (int)ti.grow0;
-            if (p.conv_cb) {  // convolution tap: shifted rows of the padded image, channel block kb % conv_cb
-              const int tap = kb / p.conv_cb;
-              arow += (tap / 3 - 1) * p.conv_w2 + (tap % 3 - 1);
-              kc = (kb % p.conv_cb) * BK;
-              seg = 0;
-            }
-            const int wpart = p.mma_n ? p.mma_n * (BK * 2 / 2) : C::W_PART;  // bytes of this CTA's half of the W tile
-            const int wrow = (ti.n_tile * NSLOT + sl_) * BN + rank * (p.mma_n ? p.mma_n / 2 : BN / 2);
-            if (rank == 0) mbar_arrive_expect_tx(&full[stage], 2 * (X3 ? 2 * A_TILE_BYTES + 2 * wpart : A_TILE_BYTES + wpart));
-            if (X3) {
-              tma_load_2d_cg2(sa, &p.a_hi[seg], kc, arow, &full[stage]);
-              tma_load_2d_cg2(sa + A_TILE_BYTES, &p.a_lo[seg], kc, arow, &full[stage]);
-              tma_load_3d_cg2(sa + 2 * A_TILE_BYTES, &p.w_hi_half, kb * BK, wrow, ti.sel, &full[stage]);
-              tma_load_3d_cg2(sa + 2 * A_TILE_BYTES + C::W_PART, &p.w_lo_half, kb * BK, wrow, ti.sel, &full[stage]);
-            } else {
-              tma_load_2d_cg2(sa, &p.a_hi[seg], kc, arow, &full[stage]);
-              tma_load_3d_cg2(sa + A_TILE_BYTES, &p.w_hi_half, kb * BK, wrow, ti.sel, &full[stage]);
-            }
+          // this CTA's A rows and its half (128 of 256 rows) of the W tile; the bytes of BOTH CTAs complete on the
+          // leader's barrier, which only the leader arms
+          const int sl_ = it / p.kb_total, kb = it % p.kb_total;  // slot outermost: slot 0 completes (and is normalised) first
+          int seg = kb >= p.kb0 ? 1 : 0;
+          int kc = (seg ? kb - p.kb0 : kb) * BK;
+          int arow = (int)ti.grow0;
+          if (p.conv_cb) {  // convolution tap: shifted rows of the padded image, channel block kb % conv_cb
+            const int tap = kb / p.conv_cb;
+            arow += (tap / 3 - 1) * p.conv_w2 + (tap % 3 - 1);
+            kc = (kb % p.conv_cb) * BK;
+            seg = 0;
+          }
+          const int wpart = p.mma_n ? p.mma_n * (BK * 2 / 2) : C::W_PART;  // bytes of this CTA's half of the W tile
+          const int wrow = (ti.n_tile * NSLOT + sl_) * BN + rank * (p.mma_n ? p.mma_n / 2 : BN / 2);
+          if (rank == 0) mbar_arrive_expect_tx(&full[stage], 2 * (X3 ? 2 * A_TILE_BYTES + 2 * wpart : A_TILE_BYTES + wpart));
+          if (X3) {
+            tma_load_2d_cg2(sa, &p.a_hi[seg], kc, arow, &full[stage]);
+            tma_load_2d_cg2(sa + A_TILE_BYTES, &p.a_lo[seg], kc, arow, &full[stage]);
+            tma_load_3d_cg2(sa + 2 * A_TILE_BYTES, &p.w_hi, kb * BK, wrow, ti.sel, &full[stage]);
+            tma_load_3d_cg2(sa + 2 * A_TILE_BYTES + C::W_PART, &p.w_lo, kb * BK, wrow, ti.sel, &full[stage]);
           } else {
-            const int pass = it / p.kb_total, kb = it % p.kb_total;
-            // pass order (x3): A_lo*W_hi, A_hi*W_lo, A_hi*W_hi ; (bf16): A_hi*W_hi
-            const bool a_lo = (p.passes == 3) && pass == 0;
-            const bool w_lo = (p.passes == 3) && pass == 1;
-            int seg = kb >= p.kb0 ? 1 : 0;
-            int kc = (seg ? kb - p.kb0 : kb) * BK;
-            int arow = (int)ti.grow0;
-            if (p.conv_cb) {
-              const int tap = kb / p.conv_cb;
-              arow += (tap / 3 - 1) * p.conv_w2 + (tap % 3 - 1);
-              kc = (kb % p.conv_cb) * BK;
-              seg = 0;
-            }
-            mbar_arrive_expect_tx(&full[stage], STAGE_BYTES);
-            tma_load_2d(sa, a_lo ? &p.a_lo[seg] : &p.a_hi[seg], kc, arow, &full[stage]);
-#pragma unroll
-            for (int sl_ = 0; sl_ < NSLOT; ++sl_)
-              tma_load_3d(sa + A_TILE_BYTES + sl_ * W_TILE_BYTES, w_lo ? &p.w_lo : &p.w_hi, kb * BK,
-                          (ti.n_tile * NSLOT + sl_) * BN, ti.sel, &full[stage]);
+            tma_load_2d_cg2(sa, &p.a_hi[seg], kc, arow, &full[stage]);
+            tma_load_3d_cg2(sa + A_TILE_BYTES, &p.w_hi, kb * BK, wrow, ti.sel, &full[stage]);
           }
         }
       }
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
-    const uint32_t idesc = make_idesc(CG2 ? 2 * BM : BM, (CG2 && p.mma_n) ? p.mma_n : BN, true);
+    const uint32_t idesc = make_idesc(2 * BM, p.mma_n ? p.mma_n : BN, true);
     int g = 0, li = 0;  // li: index among this CTA's live tiles
 #ifdef LG_TC_TRACE
     long long trm[8][4];
     const bool tracing = EPI == TEPI_LN_GELU && blockIdx.x == 0;
 #endif
-    TileWalk<MC> walk(total_tiles, n_tiles);
+    TileWalk walk(tiles, n_tiles);
     TileInfo ti;
     bool store;
-    while ((!CG2 || rank == 0) && walk.next(p, ti, store)) {  // pair mode: the leader issues for both CTAs
+    while (rank == 0 && walk.next(p, ti, store)) {  // the leader issues for both CTAs
       const int buf = NSLOT == 1 ? li % NBUF : 0;
       const uint32_t par = NSLOT == 1 ? (uint32_t)((li / NBUF) & 1) : (uint32_t)(li & 1);
-      // the epilogue warps (pair mode: of both CTAs) have drained this accumulator; the LayerNorm variant waits per
-      // slot, right before the slot's first MMA, so that slot 0 of the next tile overlaps the normalisation of slot 1
-      if (NSLOT == 1 || !CG2) {
-        for (int bb = 0; bb < (NSLOT == 1 ? 1 : 2); ++bb) {
-          if (CG2) mbar_wait_cluster(&acc_empty[buf + bb], par ^ 1, p.dbg, 20, li);
-          else mbar_wait(&acc_empty[buf + bb], par ^ 1, p.dbg, 20, li);
-        }
+      // the epilogue warps of both CTAs have drained this accumulator; the LayerNorm variant waits per slot, right
+      // before the slot's first MMA, so that slot 0 of the next tile overlaps the normalisation of slot 1
+      if (NSLOT == 1) {
+        mbar_wait_cluster(&acc_empty[buf], par ^ 1, p.dbg, 20, li);
         tc_fence_after();
       }
       const uint32_t acc = tmem_base + buf * BN;
       for (int it = 0; it < iters; ++it, ++g) {
         const int stage = g % STAGES, round = g / STAGES;
-        if (NSLOT == 2 && CG2 && it % p.kb_total == 0) {
+        if (NSLOT == 2 && it % p.kb_total == 0) {
           mbar_wait_cluster(&acc_empty[it / p.kb_total], par ^ 1, p.dbg, 20, li);
           tc_fence_after();
         }
@@ -361,47 +324,31 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
 #endif
         if (elect_one()) {
           const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES);
-          if (CG2) {
-            const int sl_ = it / p.kb_total, kb = it % p.kb_total;
-            const uint32_t d = acc + sl_ * BN;
-            if (X3) {
-              const uint64_t ahi = make_sdesc_sw128(sa), alo = make_sdesc_sw128(sa + A_TILE_BYTES);
-              const uint64_t whi = make_sdesc_sw128(sa + 2 * A_TILE_BYTES), wlo = make_sdesc_sw128(sa + 2 * A_TILE_BYTES + C::W_PART);
+          const int sl_ = it / p.kb_total, kb = it % p.kb_total;
+          const uint32_t d = acc + sl_ * BN;
+          if (X3) {
+            const uint64_t ahi = make_sdesc_sw128(sa), alo = make_sdesc_sw128(sa + A_TILE_BYTES);
+            const uint64_t whi = make_sdesc_sw128(sa + 2 * A_TILE_BYTES), wlo = make_sdesc_sw128(sa + 2 * A_TILE_BYTES + C::W_PART);
 #pragma unroll
-              for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, alo + 2 * k, whi + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
+            for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, alo + 2 * k, whi + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
 #pragma unroll
-              for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, ahi + 2 * k, wlo + 2 * k, idesc, 1u);
+            for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, ahi + 2 * k, wlo + 2 * k, idesc, 1u);
 #pragma unroll
-              for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, ahi + 2 * k, whi + 2 * k, idesc, 1u);
-            } else {
-              const uint64_t adesc = make_sdesc_sw128(sa), bdesc = make_sdesc_sw128(sa + A_TILE_BYTES);
-#pragma unroll
-              for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
-            }
-            mma_commit_cg2(&empty[stage], (uint16_t)3);  // frees the stage in both CTAs
-            if (kb == p.kb_total - 1) mma_commit_cg2(&acc_full[buf + sl_], (uint16_t)3);  // this 256-column accumulator is complete
+            for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, ahi + 2 * k, whi + 2 * k, idesc, 1u);
           } else {
-            const uint64_t adesc = make_sdesc_sw128(sa);
+            const uint64_t adesc = make_sdesc_sw128(sa), bdesc = make_sdesc_sw128(sa + A_TILE_BYTES);
 #pragma unroll
-            for (int sl_ = 0; sl_ < NSLOT; ++sl_) {
-              const uint64_t bdesc = make_sdesc_sw128(sa + A_TILE_BYTES + sl_ * W_TILE_BYTES);
-#pragma unroll
-              for (int k = 0; k < BK / 16; ++k)
-                mma_ss(acc + sl_ * BN, adesc + 2 * k, bdesc + 2 * k, idesc, (it > 0 || k > 0) ? 1u : 0u);
-            }
-            mma_commit(&empty[stage]);
-            if (it == iters - 1) {
-              mma_commit(&acc_full[buf]);
-              if (NSLOT == 2) mma_commit(&acc_full[1]);
-            }
+            for (int k = 0; k < BK / 16; ++k) mma_ss_cg2(d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
           }
+          mma_commit_cg2(&empty[stage], (uint16_t)3);  // frees the stage in both CTAs
+          if (kb == p.kb_total - 1) mma_commit_cg2(&acc_full[buf + sl_], (uint16_t)3);  // this 256-column accumulator is complete
         }
         __syncwarp();
       }
       ++li;
     }
 #ifdef LG_TC_TRACE
-    if (tracing && lane == 0 && (!CG2 || rank == 0))
+    if (tracing && lane == 0 && rank == 0)
       for (int i = 0; i < li && i < 8; ++i)
         printf("TRM tile %d slot0_free %lld slot0_last_full %lld slot1_free %lld slot1_last_full %lld\n", i, trm[i][0], trm[i][1], trm[i][2], trm[i][3]);
 #endif
@@ -431,7 +378,7 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
     long long tre[8][6];
     const bool tracing = EPI == TEPI_LN_GELU && blockIdx.x == 0 && ew == 0;
 #endif
-    TileWalk<MC> walk(total_tiles, n_tiles);
+    TileWalk walk(tiles, n_tiles);
     TileInfo ti;
     bool store;
     while (walk.next(p, ti, store)) {
@@ -440,9 +387,9 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
       auto release_acc = [&](int bb) {  // this warp has finished reading accumulator bb
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) { if (CG2) mbar_arrive_leader(&acc_empty[bb]); else mbar_arrive(&acc_empty[bb]); }
+        if (lane == 0) mbar_arrive_leader(&acc_empty[bb]);
       };
-      if (!store) {  // dead tile of a live pair (only in cluster mode): drain the accumulator(s), write nothing
+      if (!store) {  // dead tile of a live pair: drain the accumulator(s), write nothing
         for (int bb = 0; bb < (NSLOT == 1 ? 1 : 2); ++bb) {
           mbar_wait(&acc_full[buf + bb], par, p.dbg, 23, li);
           tc_fence_after();
@@ -843,7 +790,7 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
           }
           const bool f32out = NSLOT == 1 && (EPI == TEPI_RESID || EPI == TEPI_F32);
           const bool fp16 = EPI == TEPI_QKV;
-          const bool has16 = fp16 || EPI == TEPI_BF16 || EPI == TEPI_CONV || EPI == TEPI_RESID ||
+          const bool has16 = fp16 || EPI == TEPI_CONV || EPI == TEPI_RESID ||
                              (EPI == TEPI_F32 && p.out_h != nullptr);
           const bool haslo = has16 && !fp16 && p.out_l != nullptr;
           if (f32out) {
@@ -898,11 +845,8 @@ __global__ void __launch_bounds__(LinCfg<NSLOT, CG2, X3>::THREADS, 1) tc_linear_
   }
   tc_fence_before();
   __syncthreads();
-  if (MC) cluster_sync_all();  // no CTA leaves while the leader may still read its operands / arrive on its barriers
-  if (warp == 1) {
-    if (CG2) tmem_dealloc_cg2<512>(tmem_base);
-    else tmem_dealloc<512>(tmem_base);
-  }
+  cluster_sync_all();  // no CTA leaves while the leader may still read its operands / arrive on its barriers
+  if (warp == 1) tmem_dealloc_cg2<512>(tmem_base);
 }
 
 // fp32 -> bf16 hi (/ lo) for rows < len
@@ -1010,9 +954,9 @@ int amap(LgHandle* h, CUtensorMap* out, const void* base, uint64_t rows, uint64_
   mc->m.emplace(key, *out);
   return 0;
 }
-// W operand: nsel x [Nout, K] bf16, box 64 x 256 x 1
+// W operand: nsel x [Nout, K] bf16, box 64 x box_rows x 1
 int wmap(LgHandle* h, CUtensorMap* out, const void* base, uint64_t Nout, uint64_t K, uint64_t nsel, uint64_t sel_stride_elems,
-         uint32_t box_rows = BN) {
+         uint32_t box_rows) {
   MapCache* mc = static_cast<MapCache*>(h->tc.map_cache);
   MapKey key{base, Nout, K, nsel | ((uint64_t)box_rows << 32), sel_stride_elems + 2};
   auto it = mc->m.find(key);
@@ -1050,70 +994,55 @@ int omap_qk(LgHandle* h, CUtensorMap* out, const void* base, uint64_t Lp, uint64
   return 0;
 }
 
-template <int NSLOT, int EPI, bool CG2, bool X3>
+template <int NSLOT, int EPI>
 int launch_linear_t(TcLinParams& p, int n_tiles, cudaStream_t stream) {
-  using C = LinCfg<NSLOT, CG2, X3>;
-  constexpr int smem = C::SMEM;
-  if (int r = lg_func_smem_once((const void*)tc_linear_kernel<NSLOT, EPI, CG2, X3>, smem)) return r;
+  const bool x3 = p.passes == 3;
+  void (*kernel)(TcLinParams) = x3 ? tc_linear_kernel<NSLOT, EPI, true> : tc_linear_kernel<NSLOT, EPI, false>;
+  const int smem = x3 ? LinCfg<NSLOT, true>::SMEM : LinCfg<NSLOT, false>::SMEM;
+  if (int r = lg_func_smem_once((const void*)kernel, smem)) return r;
   const int num_sms = lg_num_sms();
   p.n_tiles = n_tiles;
-  const int total = n_tiles * p.st.S * (p.st.Lp / BM);
+  const int total = total_tiles(p);
   int grid = total < num_sms ? total : num_sms;
+  grid &= ~1;  // whole clusters of two (total is even)
   cudaLaunchConfig_t cfg{};
   cudaLaunchAttribute at[2];
-  unsigned na = 0;
-  if (CG2) {
-    grid &= ~1;  // whole clusters of two (total is even: S is even)
-    at[na].id = cudaLaunchAttributeClusterDimension;
-    at[na].val.clusterDim.x = 2; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  if (tc_use_pdl()) {
-    at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  cfg.attrs = at; cfg.numAttrs = na;
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(C::THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, tc_linear_kernel<NSLOT, EPI, CG2, X3>, p);
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = 2;
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(LinCfg<NSLOT, false>::THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, p);
   if (e != cudaSuccess) return lg_set_cuda_error(e, __FILE__, __LINE__);
   return 0;
 }
-template <int NSLOT, int EPI>
-int launch_linear_e(TcLinParams& p, int n_tiles, bool cg2, cudaStream_t stream) {
-  if (!cg2) return launch_linear_t<NSLOT, EPI, false, false>(p, n_tiles, stream);
-  return p.passes == 3 ? launch_linear_t<NSLOT, EPI, true, true>(p, n_tiles, stream)
-                       : launch_linear_t<NSLOT, EPI, true, false>(p, n_tiles, stream);
-}
 int launch_linear(TcLinParams& p, int n_tiles, cudaStream_t stream) {
-  static const bool use_cg2 = !(getenv("LG_TC_NO_CG2") && atoi(getenv("LG_TC_NO_CG2")) != 0);
-  // per-tile weight selection (final_proj head of the pair's exit layer; the partner's descriptors in the assignment
-  // sweeps): the two row tiles of a CTA pair share W only when both belong to the same sequence, i.e. Lp % 256 == 0
-  const bool cg2 = use_cg2 && (p.w_select == 0 || (p.st.Lp / BM) % 2 == 0);
   switch (p.epi) {
-    case TEPI_QKV: return launch_linear_e<1, TEPI_QKV>(p, n_tiles, cg2, stream);
-    case TEPI_BF16: return launch_linear_e<1, TEPI_BF16>(p, n_tiles, cg2, stream);
-    case TEPI_LN_GELU: return launch_linear_e<2, TEPI_LN_GELU>(p, 1, cg2, stream);
-    case TEPI_RESID: return launch_linear_e<1, TEPI_RESID>(p, n_tiles, cg2, stream);
-    case TEPI_F32: return launch_linear_e<1, TEPI_F32>(p, n_tiles, cg2, stream);
-    case TEPI_CONV: return launch_linear_e<1, TEPI_CONV>(p, n_tiles, cg2, stream);
-    case TEPI_LSE: return launch_linear_e<1, TEPI_LSE>(p, n_tiles, cg2, stream);
-    case TEPI_ARGMAX: return launch_linear_e<1, TEPI_ARGMAX>(p, n_tiles, cg2, stream);
+    case TEPI_QKV: return launch_linear_t<1, TEPI_QKV>(p, n_tiles, stream);
+    case TEPI_LN_GELU: return launch_linear_t<2, TEPI_LN_GELU>(p, 1, stream);
+    case TEPI_RESID: return launch_linear_t<1, TEPI_RESID>(p, n_tiles, stream);
+    case TEPI_F32: return launch_linear_t<1, TEPI_F32>(p, n_tiles, stream);
+    case TEPI_CONV: return launch_linear_t<1, TEPI_CONV>(p, n_tiles, stream);
+    case TEPI_LSE: return launch_linear_t<1, TEPI_LSE>(p, n_tiles, stream);
+    case TEPI_ARGMAX: return launch_linear_t<1, TEPI_ARGMAX>(p, n_tiles, stream);
   }
   return lg_set_error("launch_linear: bad epilogue");
 }
 
 struct LinDesc {
-  const __nv_bfloat16 *a0h, *a0l; int k0;   // segment 0
-  const __nv_bfloat16 *a1h, *a1l; int k1;   // segment 1 (k1 = 0: none)
-  size_t w_off; int nout;                   // offset (elements) into the split weight arrays
+  const __nv_bfloat16 *a0h, *a0l; int k0;   // A segment 0: [S * Lp rows, k0]
+  const __nv_bfloat16 *a1h, *a1l; int k1;   // A segment 1 (k1 = 0: none)
+  const __nv_bfloat16 *wh, *wl; int nout;   // W: nsel x [nout, K] (bf16 hi / lo)
   int nsel; size_t sel_stride;
 };
 
+// A / W tensor maps, output maps and launch of one tensor-core GEMM (linears, assignment sweeps, convolutions)
 int run_linear(LgHandle* h, const SeqState& st, const LinDesc& d, TcLinParams& p, cudaStream_t stream) {
   const bool x3 = h->cfg.precision == LG_PREC_BF16X3;
   const uint64_t rows = (uint64_t)st.S * st.Lp;
-  const int K = d.k0 + d.k1;
+  const int K = p.conv_cb ? 9 * d.k0 : d.k0 + d.k1;  // a 3x3 convolution runs K over the nine taps of one A matrix
+  const uint32_t wbox = (p.mma_n ? p.mma_n : BN) / 2;  // each CTA of a pair holds half of the W tile's rows
   int r;
   if ((r = amap(h, &p.a_hi[0], d.a0h, rows, d.k0))) return r;
   p.a_hi[1] = p.a_hi[0];
@@ -1124,14 +1053,9 @@ int run_linear(LgHandle* h, const SeqState& st, const LinDesc& d, TcLinParams& p
     p.a_lo[1] = p.a_lo[0];
     if (d.k1 && (r = amap(h, &p.a_lo[1], d.a1l, rows, d.k1))) return r;
   }
-  if ((r = wmap(h, &p.w_hi, h->tc.w_hi + d.w_off, d.nout, K, d.nsel, d.sel_stride))) return r;
+  if ((r = wmap(h, &p.w_hi, d.wh, d.nout, K, d.nsel, d.sel_stride, wbox))) return r;
   p.w_lo = p.w_hi;
-  if (x3 && (r = wmap(h, &p.w_lo, h->tc.w_lo + d.w_off, d.nout, K, d.nsel, d.sel_stride))) return r;
-  {  // half-height boxes: each CTA of a pair holds 128 of the 256 rows of a W tile
-    if ((r = wmap(h, &p.w_hi_half, h->tc.w_hi + d.w_off, d.nout, K, d.nsel, d.sel_stride, BN / 2))) return r;
-    p.w_lo_half = p.w_hi_half;
-    if (x3 && (r = wmap(h, &p.w_lo_half, h->tc.w_lo + d.w_off, d.nout, K, d.nsel, d.sel_stride, BN / 2))) return r;
-  }
+  if (x3 && (r = wmap(h, &p.w_lo, d.wl, d.nout, K, d.nsel, d.sel_stride, wbox))) return r;
   if (p.out_h && (r = omap2d(h, &p.o_h, p.out_h, 2, p.ldb, rows, 64, true))) return r;
   if (p.out_l && (r = omap2d(h, &p.o_l32, p.out_l, 2, p.ldb, rows, 32, false))) return r;
   if (p.out_h && p.epi == TEPI_LN_GELU && (r = omap2d(h, &p.o_h32, p.out_h, 2, p.ldb, rows, 32, false))) return r;
@@ -1148,7 +1072,7 @@ int run_linear(LgHandle* h, const SeqState& st, const LinDesc& d, TcLinParams& p
   if (p.w_select != 2) p.w_select = d.nsel > 1;
   p.dbg = h->tc.dbg;
   h->launches += 1;
-  return launch_linear(p, d.nout / BN, stream);
+  return launch_linear(p, (d.nout + BN - 1) / BN, stream);
 }
 }  // namespace
 
@@ -1172,24 +1096,12 @@ int tc_assign_sweeps(LgHandle* h, const TcBuffers& b, const SeqState& st, const 
     p.part = part; p.part_arg = part_arg; p.part_stride = 2 * ntc; p.term = term;
     p.logmat = sweep == 1 ? logmat : nullptr; p.mat_m = M; p.mat_n = N;
     p.w_select = 2;
-    const bool x3 = h->cfg.precision == LG_PREC_BF16X3;
-    const uint64_t rows = (uint64_t)st.S * st.Lp;
+    // W = the partner sequence's rows of p: one [Lp, 256] matrix per sequence
+    LinDesc ld{b.msgh, b.msgl, LG_DIM, nullptr, nullptr, 0, b.msgh, b.msgl, st.Lp, st.S, (size_t)st.Lp * LG_DIM};
     int r;
-    if ((r = amap(h, &p.a_hi[0], b.msgh, rows, LG_DIM))) return r;
-    p.a_hi[1] = p.a_hi[0]; p.a_lo[0] = p.a_hi[0]; p.a_lo[1] = p.a_hi[0];
-    if (x3) { if ((r = amap(h, &p.a_lo[0], b.msgl, rows, LG_DIM))) return r; p.a_lo[1] = p.a_lo[0]; }
-    if ((r = wmap(h, &p.w_hi, b.msgh, st.Lp, LG_DIM, st.S, (uint64_t)st.Lp * LG_DIM))) return r;
-    p.w_lo = p.w_hi;
-    if (x3 && (r = wmap(h, &p.w_lo, b.msgl, st.Lp, LG_DIM, st.S, (uint64_t)st.Lp * LG_DIM))) return r;
-    if ((r = wmap(h, &p.w_hi_half, b.msgh, st.Lp, LG_DIM, st.S, (uint64_t)st.Lp * LG_DIM, BN / 2))) return r;
-    p.w_lo_half = p.w_hi_half;
-    if (x3 && (r = wmap(h, &p.w_lo_half, b.msgl, st.Lp, LG_DIM, st.S, (uint64_t)st.Lp * LG_DIM, BN / 2))) return r;
-    p.kb0 = LG_DIM / BK; p.kb_total = LG_DIM / BK; p.passes = x3 ? 3 : 1;
-    p.st = st; p.dbg = h->tc.dbg;
-    h->launches += 1;
     {
       Timer tm(h, LG_K_ASSIGN_MATRIX, stream, sweep == 1 && logmat != nullptr);  // the matrix-writing sweep on its own
-      if ((r = launch_linear(p, ntc, stream))) return r;
+      if ((r = run_linear(h, st, ld, p, stream))) return r;
     }
     if (sweep == 0) {
       if ((r = misc_assign_term(a, st, part, 2 * ntc, BN / 2, term, stream))) return r;
@@ -1279,7 +1191,7 @@ int tc_input_proj(LgHandle* h, const TcBuffers& b, const SeqState& st, const flo
   TcLinParams p{};
   p.epi = TEPI_F32; p.scale = 1.f; p.bias = h->wpk + h->o_inb;
   p.out_f32 = x; p.ldo = LG_DIM; p.out_h = b.xh; p.out_l = b.xl; p.ldb = LG_DIM;
-  LinDesc ld{b.hh, b.hl, d, nullptr, nullptr, 0, h->o_inw, LG_DIM, 1, 0};
+  LinDesc ld{b.hh, b.hl, d, nullptr, nullptr, 0, h->tc.w_hi + h->o_inw, h->tc.w_lo + h->o_inw, LG_DIM, 1, 0};
   return run_linear(h, st, ld, p, stream);
 }
 
@@ -1288,7 +1200,8 @@ int tc_final_proj(LgHandle* h, const TcBuffers& b, const SeqState& st, float* p_
   p.epi = TEPI_F32; p.scale = 0.25f;  // / 256^(1/4) (lightglue.py:291)
   p.bias = h->wpk + h->o_assign + AO_FB; p.bias_sel_stride = ASSIGN_BLOB_PAD;
   p.out_f32 = p_out; p.ldo = LG_DIM; p.out_h = b.msgh; p.out_l = b.msgl; p.ldb = LG_DIM;  // bf16 images feed the sweeps
-  LinDesc ld{b.xh, b.xl, LG_DIM, nullptr, nullptr, 0, h->o_assign + AO_FW, LG_DIM, h->cfg.n_layers, ASSIGN_BLOB_PAD};
+  const size_t fw = h->o_assign + AO_FW;
+  LinDesc ld{b.xh, b.xl, LG_DIM, nullptr, nullptr, 0, h->tc.w_hi + fw, h->tc.w_lo + fw, LG_DIM, h->cfg.n_layers, ASSIGN_BLOB_PAD};
   return run_linear(h, st, ld, p, stream);
 }
 
@@ -1296,39 +1209,18 @@ int tc_conv(LgHandle* h, const SeqState& st, const __nv_bfloat16* in_h, const __
             const float* bias, int relu, int B, int H, int W, __nv_bfloat16* out_h, __nv_bfloat16* out_l, int cout, float* out_f32,
             int ldo, cudaStream_t stream) {
   const bool x3 = h->cfg.precision == LG_PREC_BF16X3;
-  const uint64_t rows = (uint64_t)st.S * st.Lp;
-  const int K = taps * cin;
   if (cin % BK != 0 || (taps != 1 && taps != 9)) return lg_set_error("tc_conv: Cin must be a multiple of 64, 1x1 or 3x3");
   TcLinParams p{};
   p.epi = out_f32 ? TEPI_F32 : TEPI_CONV;
   p.scale = 1.f; p.bias = bias; p.relu = relu;
   p.out_f32 = out_f32; p.ldo = ldo; p.out_h = out_h; p.out_l = x3 ? out_l : nullptr; p.ldb = cout;
-  int r;
-  if ((r = amap(h, &p.a_hi[0], in_h, rows, cin))) return r;
-  p.a_hi[1] = p.a_hi[0]; p.a_lo[0] = p.a_hi[0]; p.a_lo[1] = p.a_hi[0];
-  if (x3) { if ((r = amap(h, &p.a_lo[0], in_l, rows, cin))) return r; p.a_lo[1] = p.a_lo[0]; }
-  if ((r = wmap(h, &p.w_hi, h->tc.w_hi + w_off, BN, K, 1, 0))) return r;
-  p.w_lo = p.w_hi;
-  if (x3 && (r = wmap(h, &p.w_lo, h->tc.w_lo + w_off, BN, K, 1, 0))) return r;
   const int mma_n = cout <= 64 ? 64 : cout <= 128 ? 128 : BN;  // no MMA columns for the zero rows of a narrow layer
   p.mma_n = mma_n == BN ? 0 : mma_n;
-  if ((r = wmap(h, &p.w_hi_half, h->tc.w_hi + w_off, BN, K, 1, 0, mma_n / 2))) return r;
-  p.w_lo_half = p.w_hi_half;
-  if (x3 && (r = wmap(h, &p.w_lo_half, h->tc.w_lo + w_off, BN, K, 1, 0, mma_n / 2))) return r;
-  if (out_f32) {
-    if ((r = omap2d(h, &p.o_f32, out_f32, 4, ldo, rows, 32, true))) return r;
-  } else {
-    if ((r = omap2d(h, &p.o_h, out_h, 2, cout, rows, 64, true))) return r;
-    if (p.out_l && (r = omap2d(h, &p.o_l32, out_l, 2, cout, rows, 32, false))) return r;
-  }
-  p.kb0 = p.kb_total = K / BK;
-  p.passes = x3 ? 3 : 1;
-  p.st = st; p.w_select = 0; p.dbg = h->tc.dbg;
   p.conv_cb = taps == 9 ? cin / BK : 0;
   p.conv_w2 = W + 2; p.conv_h = H; p.conv_w = W;
   p.conv_plane = (long)(H + 2) * (W + 2); p.conv_rows = (long)B * p.conv_plane;
-  h->launches += 1;
-  return launch_linear(p, 1, stream);
+  LinDesc ld{in_h, in_l, cin, nullptr, nullptr, 0, h->tc.w_hi + w_off, h->tc.w_lo + w_off, BN, 1, 0};
+  return run_linear(h, st, ld, p, stream);
 }
 
 int tc_block(LgHandle* h, const TcBuffers& b, const SeqState& st, int layer, int blk, float* x, const float* cs,
@@ -1336,18 +1228,18 @@ int tc_block(LgHandle* h, const TcBuffers& b, const SeqState& st, int layer, int
   const BlockOff& o = blk == 0 ? h->bself : h->bcross;
   const size_t base = h->o_layers + (size_t)layer * h->layer_stride + (blk == 0 ? 0 : h->bself.total);
   const float* bw = h->wpk + base;
+  const __nv_bfloat16 *wh = h->tc.w_hi + base, *wl = h->tc.w_lo + base;
   // Tile order against the 126 MB L2: every kernel of the chain reads what its predecessor wrote, and only the part written
   // LAST is still resident.  QKV and ffn.0 walk their tile lists backwards, ffn.3 (and the attention grid) forwards: ffn.3
   // starts on the hidden tiles ffn.0 finished with, the next QKV on the x images ffn.3 finished with, attention on the
   // q / k / v of the sequences QKV wrote last, ffn.0 on the context of the sequences attention wrote last.
-  static const bool no_rev = getenv("LG_TC_NO_REVERSE") && atoi(getenv("LG_TC_NO_REVERSE")) != 0;
   {  // QKV (+RoPE) / [to_qk | to_v] projection
     Timer t(h, LG_K_LINEAR, stream);
     Timer t2(h, LG_K_QKV, stream);
     TcLinParams p{};
-    p.epi = TEPI_QKV; p.rope = blk == 0; p.scale = 1.f; p.bias = bw + o.bp; p.reverse = no_rev ? 0 : 1;
+    p.epi = TEPI_QKV; p.rope = blk == 0; p.scale = 1.f; p.bias = bw + o.bp; p.reverse = 1;
     p.q = b.q; p.k = b.k; p.vt = b.vt; p.cs = cs;
-    LinDesc ld{b.xh, b.xl, LG_DIM, nullptr, nullptr, 0, base + o.wp, blk == 0 ? 3 * LG_DIM : 2 * LG_DIM, 1, 0};
+    LinDesc ld{b.xh, b.xl, LG_DIM, nullptr, nullptr, 0, wh + o.wp, wl + o.wp, blk == 0 ? 3 * LG_DIM : 2 * LG_DIM, 1, 0};
     int r = run_linear(h, st, ld, p, stream);
     if (r) return r;
   }
@@ -1357,22 +1249,13 @@ int tc_block(LgHandle* h, const TcBuffers& b, const SeqState& st, int layer, int
     if (r) return r;
   }
   Timer t(h, LG_K_LINEAR, stream);
-  static const bool no_fold = getenv("LG_TC_NO_FOLD") && atoi(getenv("LG_TC_NO_FOLD")) != 0;  // debug: separate out_proj launch
-  if (no_fold) {  // out_proj / to_out -> msg
-    TcLinParams p{};
-    p.epi = TEPI_BF16; p.scale = 1.f; p.bias = bw + o.bo; p.out_h = b.msgh; p.out_l = b.msgl; p.ldb = LG_DIM;
-    LinDesc ld{b.ctxh, b.ctxl, LG_DIM, nullptr, nullptr, 0, base + o.wo, LG_DIM, 1, 0};
-    int r = run_linear(h, st, ld, p, stream);
-    if (r) return r;
-  }
   {  // ffn.0 on cat([x, msg]) + LayerNorm + GELU -> h; the output projection is folded into the weights (W1f, b1f:
      // lg_handle.h), so the GEMM reads cat([x, ctx]) and `msg` is never formed
     TcLinParams p{};
-    p.epi = TEPI_LN_GELU; p.scale = 1.f; p.bias = bw + (no_fold ? o.b1 : o.b1f); p.ln_g = bw + o.g; p.ln_b = bw + o.be;
-    p.reverse = no_rev ? 0 : 1;
+    p.epi = TEPI_LN_GELU; p.scale = 1.f; p.bias = bw + o.b1f; p.ln_g = bw + o.g; p.ln_b = bw + o.be;
+    p.reverse = 1;
     p.out_h = b.hh; p.out_l = b.hl; p.ldb = LG_FFN;
-    LinDesc ld{b.xh, b.xl, LG_DIM, no_fold ? b.msgh : b.ctxh, no_fold ? b.msgl : b.ctxl, LG_DIM, base + (no_fold ? o.w1 : o.w1f),
-               LG_FFN, 1, 0};
+    LinDesc ld{b.xh, b.xl, LG_DIM, b.ctxh, b.ctxl, LG_DIM, wh + o.w1f, wl + o.w1f, LG_FFN, 1, 0};
     Timer t2(h, LG_K_FFN0, stream);
     int r = run_linear(h, st, ld, p, stream);
     if (r) return r;
@@ -1381,7 +1264,7 @@ int tc_block(LgHandle* h, const TcBuffers& b, const SeqState& st, int layer, int
     TcLinParams p{};
     p.epi = TEPI_RESID; p.scale = 1.f; p.bias = bw + o.b2; p.out_f32 = x; p.ldo = LG_DIM;
     p.out_h = b.xh; p.out_l = b.xl; p.ldb = LG_DIM;
-    LinDesc ld{b.hh, b.hl, LG_FFN, nullptr, nullptr, 0, base + o.w2, LG_DIM, 1, 0};
+    LinDesc ld{b.hh, b.hl, LG_FFN, nullptr, nullptr, 0, wh + o.w2, wl + o.w2, LG_DIM, 1, 0};
     Timer t2(h, LG_K_FFN3, stream);
     int r = run_linear(h, st, ld, p, stream);
     if (r) return r;

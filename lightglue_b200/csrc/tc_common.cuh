@@ -7,7 +7,6 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 namespace tc {
 
@@ -252,23 +251,7 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
 // global memory a predecessor writes; both are no-ops in a plain launch.
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-// host: launch attribute for such kernels (LG_NO_PDL=1 falls back to plain stream order)
-inline bool tc_use_pdl() {
-  static const bool on = !(getenv("LG_NO_PDL") && atoi(getenv("LG_NO_PDL")) != 0);
-  return on;
-}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
-      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]),
-      "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]),
-      "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
-      : "memory");
-}
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ---------------------------------------------------------------- descriptors
@@ -285,8 +268,6 @@ __device__ __forceinline__ uint64_t make_sdesc_sw128(uint32_t smem_addr) {
   d |= (uint64_t)2 << 61;
   return d;
 }
-// advance a K-major SW128 descriptor by `k_elems` 16-bit elements along K inside the 64-element atom
-__device__ __forceinline__ uint64_t sdesc_advance_k(uint64_t d, int k_elems) { return d + (uint64_t)((k_elems * 2) >> 4); }
 
 // Instruction descriptor, kind::f16, fp32 accumulate, both operands K-major.
 //   [4,6) D format (1 = f32) | [7,10) A format | [10,13) B format (0 = f16, 1 = bf16) | [15] A major | [16] B major

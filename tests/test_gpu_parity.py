@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from lightglue_b200 import LightGlue, synth
+from lightglue_b200.ragged import pad_pairs, split_outputs
 from oracle import lightglue_oracle as oracle
 from tests.helpers import ALL_CASES, compare_outputs, forward_kwargs, load_case
 
@@ -231,6 +232,26 @@ def test_batched_early_exit_is_decided_per_pair(prec):
     for i, r in enumerate(refs):
         assert torch.equal(out["matches0"][i].cpu(), r["matches0"][0]) and torch.equal(out["matches1"][i].cpu(), r["matches1"][0])
         assert float((out["matching_scores0"][i].cpu() - r["matching_scores0"][0]).abs().max()) < 1e-3
+
+
+def test_batched_early_exit_with_odd_tile_count():
+    """Pairs that exit at different layers in one tensor-core batch whose padded length is an odd number of 128-row tiles
+    (the three pairs above and a 300-point pair: Lp = 384, three tiles).  final_proj takes the head of each pair's own exit
+    layer and the assignment sweeps the pair's own partner, so a CTA pair must never hold tiles of two sequences: every
+    pair returns its own B = 1 result."""
+    sd = synth.make_state_dict(adaptive=True, seed=2)
+    pairs = [synth.make_pair(n, b=1, seed=s)[0] for n, s in ((192, 41), (192, 41), (192, 42), (300, 43))]
+    refs = [oracle.forward(sd, p, depth_confidence=0.95, width_confidence=-1) for p in pairs]
+    assert [int(r["stop"]) for r in refs] == [6, 6, 9, 6]
+    m = LightGlue(features=None, precision="bf16x3", depth_confidence=0.95, width_confidence=-1)
+    m.load_state_dict(sd, strict=False)
+    m = m.cuda()
+    data = pad_pairs([to_cuda(p) for p in pairs])
+    out = m(data)
+    assert out["stops"] == [6, 6, 9, 6]
+    for got, r in zip(split_outputs(out, data["image0"]["num_keypoints"], data["image1"]["num_keypoints"]), refs):
+        assert torch.equal(got["matches0"].cpu(), r["matches0"]) and torch.equal(got["matches1"].cpu(), r["matches1"])
+        assert float((got["matching_scores0"].cpu() - r["matching_scores0"]).abs().max()) < 1e-3
 
 
 def test_pruned_to_zero_points_ends_the_pair_like_the_reference():

@@ -10,8 +10,8 @@ for prec in ("bf16", "bf16x3", "fp32"):
         kw = {} if adaptive else dict(depth_confidence=-1, width_confidence=-1)
         m = LightGlue(features=None, precision=prec, **kw); m.load_state_dict(sd, strict=False); m = m.cuda()
         m.pruning_keypoint_thresholds = dict(LightGlue.pruning_keypoint_thresholds, flash=-1)
-        # (300, 200): three 128-row tiles per sequence -> the assignment sweeps run one CTA per tile;
-        # (512, 512): an even number of tiles -> every tensor-core kernel runs on CTA pairs (cta_group::2)
+        # (300, 200): three 128-row tiles per sequence -> final_proj and the assignment sweeps give every sequence a
+        # fourth, dead row slot, so that no CTA pair straddles two sequences; (512, 512): an even number of tiles
         for n, mm in ((300, 200), (512, 512)):
             d, _ = synth.make_pair(n, m=mm, b=2, seed=5)
             out = m({k: {kk: vv.cuda() for kk, vv in v.items()} for k, v in d.items()})
